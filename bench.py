@@ -3,6 +3,7 @@
 
     python bench.py --gpus N --steps K --warmup W          (N>1: launched under torchrun)
     python bench.py --impl reference ...                   (the reference's CPU algorithm)
+    python bench.py ... --dump-outputs DIR                 (also save the last step's outputs)
 
 A step = one pass of the hot path (prologue + class-tile gather, one launch -> fused mask expand)
 over one batch of synthetic detections: BASELINE.json configs[1], 32 distinct images of
@@ -345,6 +346,47 @@ def _bytesum(torch, t, chunk=1 << 28):
     return sum(int(c.sum(dtype=torch.int64).item()) for c in t.split(chunk)) if t.numel() else 0
 
 
+DUMP_PIXELS_PER_IMAGE = 2048     # canvas positions per image whose mask values --dump-outputs keeps
+DUMP_MAX_BYTES = 64 << 20
+
+
+def dump_outputs(out_dir, eng, n_images):
+    """--dump-outputs: what the last timed step returned, as DIR/<name>.npy, so that two builds
+    can be compared output for output on the same seeded inputs.  Per kept instance, in image
+    order: boxes, class ids, scores and the mask's pixel count, all complete.  The masks
+    themselves (3.4 GB per step) are sampled: the values of every kept mask at
+    DUMP_PIXELS_PER_IMAGE positions per image, drawn with a fixed seed from the image's H x W."""
+    import numpy as np
+    import torch
+
+    counts = eng.d_counts[:n_images].cpu().numpy()
+    boxes = eng.d_boxes[:n_images].cpu().numpy()
+    class_ids = eng.d_class_ids[:n_images].cpu().numpy()
+    scores = eng.d_scores[:n_images].cpu().numpy()
+    kept = lambda a: np.concatenate([a[b, :k] for b, k in enumerate(counts)])  # noqa: E731
+    rng = np.random.default_rng(SEED)
+    areas, samples = [], []
+    for b, k in enumerate(counts):
+        m = eng.canvas_view(b, int(k))                     # uint8 [H, W, k] on the device
+        h, w = m.shape[:2]
+        areas.append(m.sum(dim=(0, 1), dtype=torch.int64).cpu().numpy())
+        pix = torch.from_numpy(rng.integers(0, h * w, DUMP_PIXELS_PER_IMAGE)).to(m.device)
+        samples.append(m.reshape(h * w, int(k))[pix].cpu().numpy().ravel())
+    out = {
+        "counts": counts.astype(np.float64),
+        "boxes": kept(boxes).astype(np.float64),
+        "class_ids": kept(class_ids).astype(np.float64),
+        "scores": kept(scores).astype(np.float32),
+        "mask_pixel_counts": np.concatenate(areas).astype(np.float64),
+        "mask_samples": np.concatenate(samples).astype(np.float32),
+    }
+    total = sum(a.nbytes for a in out.values())
+    assert total <= DUMP_MAX_BYTES, f"--dump-outputs would write {total} bytes"
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in out.items():
+        np.save(os.path.join(out_dir, name + ".npy"), a)
+
+
 def gather_section(ctx, eng, d_det, d_msk, n_images, masks_total, layout_note, chunks=4, reps=3):
     """One step + the gather of every rank's output to rank 0, both layouts, both transports.
     Returns the `gather` dict.  Rank 0's NVLink ingress bounds all of them: (world-1)/world of
@@ -584,6 +626,8 @@ def run_ours(args, rank, world, local_rank):
     barrier()
     total_masks = ctx.sum_over_ranks(masks_per_step)
     value = total_masks * args.steps / (max_ms * 1e-3)
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, eng, BATCH)     # before later sections reuse the buffers
 
     # ---- parity of the timed step's output: image 0 of this very batch against the oracle
     # (outside timing; rank 0; the same check tests/test_gpu_unmold.py runs exhaustively)
@@ -794,7 +838,13 @@ def main():
     ap.add_argument("--no-config4", action="store_true")
     ap.add_argument("--no-numa-bind", action="store_true")
     ap.add_argument("--cpu-procs", type=int, default=0, help="worker processes of the CPU legs")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write rank 0's outputs of the last timed step to DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs dumps the device path's outputs; the reference arm has none")
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))
