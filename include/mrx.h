@@ -17,6 +17,7 @@
  *   mrx_pack_masks         (extension: bit-packed transport of the masks of serve.py:147)
  *   mrx_mask_expand_packed (extension: the expand step writing that packed layout directly)
  *   mrx_rle_count / _write (extension: the same masks as COCO run-length encodings)
+ *   mrx_contours_count / _write <- the contour polygons display_instances traces  serve.py:160-169
  *   mrx_peer_*             (multi-GPU: the final gather of the masks to rank 0, SURVEY.md 8e)
  *
  * Conventions
@@ -38,7 +39,7 @@
 extern "C" {
 #endif
 
-#define MRX_ABI_VERSION 5
+#define MRX_ABI_VERSION 6
 
 #define MRX_OK              0
 #define MRX_E_INVALID      -1   /* bad argument (null pointer, size out of range) */
@@ -252,6 +253,56 @@ int mrx_rle_write(const float *d_tiles, const int *d_tile_index, const int *d_bo
                   const int *d_counts, const int *d_geom, int *d_col_count,
                   long long *d_inst_off, unsigned int *d_positions, unsigned int *d_run_lengths,
                   int B, int R, int mh, int mw, int max_w, void *stream);
+
+/* ---------------------------------------------------------------- contour polygons (f5) */
+/* The outline step of visualize.display_instances (serve.py:160-169): for every instance,
+ *     padded = zeros((H+2, W+2)); padded[1:-1, 1:-1] = mask
+ *     [np.fliplr(v) - 1 for v in skimage.measure.find_contours(padded, 0.5)]
+ * (fully_connected='low', positive_orientation='low'), computed from the bit-packed masks:
+ * image b at d_packed + d_packed_off[b] as uint8 [N_b, H_b, ceil(W_b/8)] (the layout of
+ * mrx_mask_expand_packed / mrx_pack_masks / np.packbits; bits past W_b are ignored).  A mask is
+ * read as zero outside its box d_boxes[b][k] (y1, x1, y2, x2) -- only the box's cells and one ring
+ * around them are scanned; an instance k >= d_counts[b] or with an empty box has no contours.
+ *
+ * Marching squares: cell (r, c) of the padded mask P is (ul, ur, ll, lr) = P[r..r+1, c..c+1],
+ * case = ul + 2 ur + 4 ll + 8 lr; segments (from, to) between edge midpoints top (r, c+1/2),
+ * bottom (r+1, c+1/2), left (r+1/2, c), right (r+1/2, c+1), cells in row-major order:
+ *     1 (T,L)  2 (R,T)  3 (R,L)  4 (L,B)  5 (T,B)  6 (R,T),(L,B)  7 (R,B)
+ *     8 (B,R)  9 (T,L),(B,R)  10 (B,T)  11 (B,L)  12 (L,R)  13 (T,R)  14 (L,T)
+ * Every edge midpoint has one segment in and one out, so the segments form cycles.  Each cycle
+ * is one polygon: it starts at the `to` point of the cycle's last-emitted segment, follows the
+ * segments and repeats its start point at the end; polygons are ordered by the emission index
+ * of each cycle's first-emitted segment.  This is the order and the start vertex skimage's
+ * contour assembly produces.  Islands run counter-clockwise in (x, y) with y down (positive
+ * shoelace area), holes the other way.  Vertices are exact halves (float32).
+ *
+ * Two calls around one host read, like the RLE pair:
+ *   mrx_contours_count:  d_row_seg [B, R, max_h+1] int32 scratch (kept for the write call);
+ *                        d_seg_off [B*R+1] int64: on return (stream-ordered) d_seg_off[i] = number
+ *                        of segments S of all instances before i = b*R + k, d_seg_off[B*R] = T.
+ *   mrx_contours_write:  total_segments = T as read back;  with  o_i = d_seg_off[i]:
+ *     d_scratch        int32 [2*T]                    (successor and end point of every segment)
+ *     d_vertices       float32 [T + T/4, 2] (x, y)    instance i's polygons, one after the other,
+ *                                                     from vertex o_i + o_i/4 (integer division)
+ *     d_contour_len    int32 [T/4]                    vertices per polygon (closing one included),
+ *                                                     instance i's from o_i/4
+ *     d_inst_contours  int32 [B*R]                    number of polygons of instance i
+ *   A cycle has at least 4 segments, so instance i has at most S_i/4 polygons and S_i + S_i/4
+ *   vertices: the regions above never overlap.  (d_scratch / d_vertices / d_contour_len may be
+ *   NULL when T == 0.)
+ * Limits: max_h, max_w (largest H_b / W_b of the batch) <= MRX_CONTOUR_MAX_DIM
+ * (MRX_E_UNSUPPORTED otherwise): the doubled padded coordinates fit 16 bits and an instance's
+ * segment count (at most 2 (H+1)(W+1)) fits 31. */
+#define MRX_CONTOUR_MAX_DIM 32766
+int mrx_contours_count(const unsigned char *d_packed, const long long *d_packed_off,
+                       const int *d_boxes, const int *d_counts, const int *d_geom,
+                       int *d_row_seg, long long *d_seg_off, int B, int R, int max_h, int max_w,
+                       void *stream);
+int mrx_contours_write(const unsigned char *d_packed, const long long *d_packed_off,
+                       const int *d_boxes, const int *d_counts, const int *d_geom,
+                       int *d_row_seg, const long long *d_seg_off, int *d_scratch,
+                       float *d_vertices, int *d_contour_len, int *d_inst_contours,
+                       long long total_segments, int B, int R, int max_h, int max_w, void *stream);
 
 /* ---------------------------------------------------------------- multi-GPU gather (8e) */
 /* Peer-memory plumbing for the final gather of the canvases to rank 0 (one process per GPU).

@@ -23,7 +23,7 @@ MRX_ST_CLASS_RANGE = 1
 MRX_ST_BOX_RANGE = 2
 MRX_GEOM_INTS = 8
 MRX_MAX_BATCH = 4096
-ABI_VERSION = 5
+ABI_VERSION = 6
 MRX_SCHED_WORDS = 4
 MRX_PEER_HANDLE_BYTES = 64
 
@@ -55,6 +55,9 @@ SIGNATURES = {
                                     _vp]),
     "mrx_rle_count": (_i, [_vp, _vp, _vp, _vp, _vp, _vp, _vp, _i, _i, _i, _i, _i, _vp]),
     "mrx_rle_write": (_i, [_vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _i, _i, _i, _i, _i, _vp]),
+    "mrx_contours_count": (_i, [_vp, _vp, _vp, _vp, _vp, _vp, _vp, _i, _i, _i, _i, _vp]),
+    "mrx_contours_write": (_i, [_vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp,
+                                C.c_longlong, _i, _i, _i, _i, _vp]),
     "mrx_peer_alloc": (_i, [C.c_ulonglong, C.POINTER(C.c_void_p)]),
     "mrx_peer_free": (_i, [_vp]),
     "mrx_peer_export": (_i, [_vp, C.c_char_p]),

@@ -9,7 +9,8 @@ NumPy value semantics, computed by the sm_100a kernels in libmrx.so.
 
 Plus batched entry points the reference lacks (it is hard-wired to one image per call,
 serve.py:48): `unmold_detections_batch`, `unmold_detections_packed_batch`,
-`unmold_detections_rle_batch`, `unmold_overlay_batch`.
+`unmold_detections_rle_batch`, `unmold_overlay_batch`, and `unmold_detections_contours_batch`
+(the contour polygons of the reference's `display_instances`, serve.py:160-169).
 
 Numerical contract (checked by tests/ against the float64 oracle): N, boxes, class ids and
 scores are bit-exact.  The mask resize runs in float32 on exact integer source coordinates;
@@ -362,6 +363,32 @@ def unmold_detections_rle_batch(items):
                          "counts": runs[int(off[i]) + i:int(off[i + 1]) + i + 1].copy()})
         out.append(metas[b] + (rles,))
     return out
+
+
+def unmold_detections_contours_batch(items):
+    """The mask outlines of the reference's `visualize.display_instances` (serve.py:160-169),
+    not an output of `unmold_detections`: for every kept instance, the contour polygons it
+    hands to matplotlib's `Polygon` -- find_contours(mask padded by one zero pixel, 0.5), as
+    (x, y) vertices without the padding.  Computed on the device from the tiles (packed expand,
+    no byte canvas, then `mrx_contours_*`); only the polygons travel to the host.
+
+    items as for `unmold_detections_batch`.  Returns a list of (boxes, class_ids, scores,
+    contours) with contours[k] the list of float64 [K, 2] arrays of instance k, each closed
+    (first row == last row), in skimage's order and with its start vertices."""
+    if len(items) == 0:
+        return []
+    with _Staged(items, canvas=False) as st:
+        eng = st.eng
+        if eng.mw > 30:
+            eng.plan(st.geoms, canvas=True)
+            eng.enqueue(st.d_det, st.d_msk)
+            dc = eng.enqueue_contours(source="canvas")
+        else:
+            eng.enqueue_packed(st.d_det, st.d_msk)
+            dc = eng.enqueue_contours()
+        counts, metas = st.meta()
+        polys = dc.to_host(counts)
+    return [metas[b] + (polys[b],) for b in range(st.n)]
 
 
 def unmold_overlay_batch(items, images, colors=None, alpha=0.5):

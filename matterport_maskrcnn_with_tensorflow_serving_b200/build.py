@@ -22,7 +22,7 @@ CSRC = os.path.join(PKG_DIR, "csrc")
 LIB_DIR = os.path.join(PKG_DIR, "lib")
 
 SOURCES = ["capi.cu", "anchors.cu", "unmold.cu", "expand_team.cu", "expand_bits.cu", "mold.cu",
-           "composite.cu", "pack.cu", "rle.cu", "peer.cu"]
+           "composite.cu", "pack.cu", "rle.cu", "contours.cu", "peer.cu"]
 HEADERS = [os.path.join(CSRC, "common.cuh"), os.path.join(CSRC, "expand.cuh"),
            os.path.join(os.path.dirname(PKG_DIR), "include", "mrx.h")]
 

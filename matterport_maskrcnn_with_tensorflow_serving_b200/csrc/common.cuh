@@ -63,6 +63,9 @@ struct SmemCache {
 };
 int ensure_dynamic_smem(const void *func, SmemCache *cache, int device, int bytes);
 
+// Exclusive scan of d[0..n) in place on `stream`, d[n] = the total (one CTA; rle.cu).
+int exclusive_scan_i64(long long *d, int n, cudaStream_t stream);
+
 // ---------------------------------------------------------------- device: PTX wrappers
 #if defined(__CUDACC__)
 

@@ -290,6 +290,12 @@ rle_counts_kernel(const unsigned int *__restrict__ positions, const long long *_
 
 }  // namespace rle
 
+int exclusive_scan_i64(long long *d, int n, cudaStream_t stream) {
+  rle::rle_offsets_kernel<<<1, 1024, 0, stream>>>(d, n);
+  MRX_LAUNCH_CHECK("rle_offsets_kernel");
+  return MRX_OK;
+}
+
 }  // namespace mrx
 
 using namespace mrx;
@@ -337,9 +343,7 @@ extern "C" int mrx_rle_count(const float *d_tiles, const int *d_tile_index, cons
   MRX_LAUNCH_CHECK("rle_walk_kernel<count>");
   rle::rle_scan_kernel<<<dim3(R, B), 256, 0, st>>>(prm);
   MRX_LAUNCH_CHECK("rle_scan_kernel");
-  rle::rle_offsets_kernel<<<1, 1024, 0, st>>>(d_inst_off, B * R);
-  MRX_LAUNCH_CHECK("rle_offsets_kernel");
-  return MRX_OK;
+  return exclusive_scan_i64(d_inst_off, B * R, st);
 }
 
 extern "C" int mrx_rle_write(const float *d_tiles, const int *d_tile_index, const int *d_boxes,

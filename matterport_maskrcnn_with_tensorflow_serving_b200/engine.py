@@ -306,6 +306,24 @@ class UnmoldEngine:
                                        self.mw, max_w, st), "mrx_rle_write")
         return d_runs, off
 
+    def enqueue_contours(self, stream=None, source="packed"):
+        """The contour polygons `display_instances` traces for every mask of the planned batch
+        (mrx_contours_count / _write), from the engine's bit-packed masks.  source="packed": the
+        packed buffer is already written (`enqueue_expand_packed` / `pack_masks`);
+        source="canvas": bit-pack the byte canvas first (`pack_masks`).  Synchronises once, to
+        size the output.  Returns a `DeviceContours`."""
+        if source not in ("packed", "canvas"):
+            raise ValueError("source: 'packed' or 'canvas'")
+        if source == "canvas":
+            self.pack_masks(stream)
+        if self.d_packed is None:
+            raise RuntimeError("no packed masks: run enqueue_expand_packed or pack_masks first")
+        n = self._n_images
+        g = self._geom_host
+        return contours_device(self.lib, self.device, self.d_packed, self.d_packed_off,
+                               self.d_boxes, self.d_counts, self.d_geom, n, self.R,
+                               int(g[:, 0].max()), int(g[:, 1].max()), stream)
+
     def pack_masks(self, stream=None):
         """EXTENSION: bit-pack the byte canvases already written for the planned batch
         (mrx_pack_masks; same output layout as `enqueue_expand_packed`).  Returns
@@ -350,6 +368,66 @@ class UnmoldEngine:
             raise ValueError(f"image {b}: a detection box falls outside the original image; "
                              "the reference's mask paste cannot broadcast it")
         return counts, hb[:n].numpy(), hk[:n].numpy(), hsc[:n].numpy()
+
+
+class DeviceContours:
+    """Output of mrx_contours_write for B images of R instance slots (layout: include/mrx.h).
+    seg_off: int64 ndarray [B*R+1] (host copy of the segment offsets); vertices float32
+    [T + T/4, 2], contour_len int32 [T/4], inst_contours int32 [B*R] (CUDA tensors)."""
+
+    def __init__(self, seg_off, vertices, contour_len, inst_contours, R):
+        self.seg_off = seg_off
+        self.vertices = vertices
+        self.contour_len = contour_len
+        self.inst_contours = inst_contours
+        self.R = R
+
+    def to_host(self, counts):
+        """Download (one synchronisation) and split: for image b, a list of counts[b] lists of
+        float64 [K, 2] (x, y) arrays -- the polygons of each instance, each closed."""
+        torch = _torch()
+        st = torch.cuda.current_stream()
+        h = [t.to("cpu", non_blocking=True) for t in (self.vertices, self.contour_len,
+                                                       self.inst_contours)]
+        st.synchronize()
+        vert, lens, ncont = (t.numpy() for t in h)
+        vert = vert.reshape(-1, 2)
+        out = []
+        for b, n in enumerate(counts):
+            per_image = []
+            for k in range(int(n)):
+                i = b * self.R + k
+                o = int(self.seg_off[i])
+                ls = lens[o // 4:o // 4 + int(ncont[i])]
+                ends = np.cumsum(ls)
+                base = o + o // 4
+                per_image.append([vert[base + e - l:base + e].astype(np.float64)
+                                  for l, e in zip(ls.tolist(), ends.tolist())])
+            out.append(per_image)
+        return out
+
+
+def contours_device(lib, device, d_packed, d_packed_off, d_boxes, d_counts, d_geom, B, R,
+                    max_h, max_w, stream=None):
+    """mrx_contours_count, one host read of the segment offsets, mrx_contours_write.  Inputs
+    are device tensors in the layouts of include/mrx.h; returns a `DeviceContours`."""
+    torch = _torch()
+    st = N.stream_ptr(stream)
+    d_rows = torch.empty((B * R * (max_h + 1),), dtype=torch.int32, device=device)
+    d_off = torch.empty((B * R + 1,), dtype=torch.int64, device=device)
+    common = (_ptr(d_packed), _ptr(d_packed_off), _ptr(d_boxes), _ptr(d_counts), _ptr(d_geom),
+              _ptr(d_rows), _ptr(d_off))
+    N.check(lib.mrx_contours_count(*common, B, R, max_h, max_w, st), "mrx_contours_count")
+    off = d_off.cpu().numpy()              # the one synchronisation: how many segments there are
+    T = int(off[-1])
+    d_scratch = torch.empty((max(2 * T, 1),), dtype=torch.int32, device=device)
+    d_vert = torch.empty((T + T // 4, 2), dtype=torch.float32, device=device)
+    d_len = torch.empty((max(T // 4, 1),), dtype=torch.int32, device=device)
+    d_ncont = torch.empty((B * R,), dtype=torch.int32, device=device)
+    N.check(lib.mrx_contours_write(*common, _ptr(d_scratch), _ptr(d_vert), _ptr(d_len),
+                                   _ptr(d_ncont), C.c_longlong(T), B, R, max_h, max_w, st),
+            "mrx_contours_write")
+    return DeviceContours(off, d_vert, d_len[:T // 4], d_ncont, R)
 
 
 class AnchorGenerator:

@@ -8,8 +8,9 @@ This module does the blending part -- the only part that touches every mask byte
 `mrx_composite_masks`, either on masks the caller holds as NumPy arrays (`apply_masks`,
 `display_instances`) or directly on the device canvas of an `UnmoldEngine`
 (`composite_batch`), which avoids the 105 MB per image device -> host copy of the masks
-when only the overlay is wanted.  Boxes, captions and contours are NOT drawn (matplotlib
-rendering is out of scope, DESIGN.md section 7).
+when only the overlay is wanted.  The contour polygons are computed on the device too
+(`mask_contours`, `api_utils.unmold_detections_contours_batch`), but boxes, captions and
+polygons are NOT drawn (matplotlib rendering is out of scope, DESIGN.md section 7).
 """
 from __future__ import annotations
 
@@ -144,6 +145,43 @@ def apply_masks(image, boxes, masks, colors, alpha=0.5):
         _ptr(d_off), _ptr(d_tab), C.c_double(1 - alpha), _ptr(d_out), 1, n,
         C.c_longlong(H * W), N.stream_ptr(None)), "mrx_composite_masks")
     return d_out.cpu().numpy()
+
+
+def mask_contours(masks, boxes=None):
+    """NumPy in, NumPy out: the outline step of `display_instances` for masks the caller holds.
+
+    masks: bool [H, W, N] (the layout `unmold_detections` returns); boxes: [N, 4] int
+    (y1, x1, y2, x2) -- a mask is read as zero outside its box, and only the box plus one ring
+    of pixels is scanned; None = the whole image.  The masks are bit-packed on the host (1/8 of
+    the bytes go to the device) and traced by `mrx_contours_*`.  Returns a list of N lists of
+    float64 [K, 2] (x, y) arrays, each closed: for instance i, what
+    find_contours(mask padded by one zero pixel, 0.5) gives, as `np.fliplr(verts) - 1`."""
+    import torch
+
+    from .engine import contours_device
+
+    N.require_cuda()
+    lib = N.load()
+    masks = np.asarray(masks)
+    if masks.ndim != 3:
+        raise ValueError(f"masks must be [H, W, N], got {masks.shape}")
+    H, W, n = masks.shape
+    if n == 0:
+        return []
+    if boxes is None:
+        boxes = np.tile(np.array([[0, 0, H, W]], np.int32), (n, 1))
+    boxes = np.ascontiguousarray(boxes, dtype=np.int32)
+    if boxes.shape != (n, 4):
+        raise ValueError(f"boxes must be [{n}, 4], got {boxes.shape}")
+    dev = torch.device("cuda", torch.cuda.current_device())
+    packed = np.packbits(np.ascontiguousarray(masks.transpose(2, 0, 1)).astype(np.bool_), axis=-1)
+    d_packed = torch.from_numpy(packed.reshape(-1)).to(dev)
+    d_off = torch.zeros(1, dtype=torch.int64, device=dev)
+    d_counts = torch.tensor([n], dtype=torch.int32, device=dev)
+    d_geom = torch.tensor([[H, W, H, W, 0, 0, H, W]], dtype=torch.int32, device=dev)
+    d_boxes = torch.from_numpy(boxes).to(dev)
+    dc = contours_device(lib, dev, d_packed, d_off, d_boxes, d_counts, d_geom, 1, n, H, W)
+    return dc.to_host([n])[0]
 
 
 def display_instances(image, boxes, masks, class_ids=None, class_names=None, scores=None,
